@@ -6,12 +6,14 @@ One "step" = one pass of the hot path over one batch: BATCH independent 2^20-poi
 NTTs (code/ntt.py:3-18) resident in HBM (BATCH * 16 MiB = 256 MiB > the 126 MB L2, so every
 step streams from HBM).  butterflies := (n/2) * log2 n per transform.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 N > 1: one process per GPU, every rank transforms its own batch (weak scaling, no data-path
 collective); time is the max over ranks.  --impl reference times the CPU oracle port
 (oracle/stark_oracle.c, all host threads) on the same workload definition.
+--dump-outputs DIR writes a fixed sample of rank 0's last timed step (see dump_outputs) so that
+two builds can be compared output for output; the inputs are seeded, so they are the same every run.
 """
 import argparse
 import ctypes
@@ -24,6 +26,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ next to the imported modules
 for _p in (os.path.join(ROOT, "stark-anatomy_b200"), os.path.join(ROOT, "oracle"), ROOT):
     if _p not in sys.path:
         sys.path.insert(0, _p)
@@ -38,6 +41,7 @@ FRI_ROUNDS = 12                 # Fri(ef 4, 64 colinearity tests).num_rounds() a
 FRI_COMPRESSIONS = 4193268      # leaves + inner nodes of the 12 trees (SURVEY 8d)
 FRI_ALG_BYTES = 50315264        # sum_r 16 N_r read + 8 N_r folded written (SURVEY 8d)
 WORKLOAD = "batch of %d independent 2^20-point forward NTTs over p=1+407*2^119 (configs[1] size, batched)" % BATCH
+DUMP_SAMPLE = 1 << 20           # residues written by --dump-outputs: 32 MiB of limbs + 8 MiB of indices
 
 
 def config_dict(world):
@@ -94,6 +98,20 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(smax) if smax else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(out_dir, y):
+    """Write a fixed, seeded sample of the batch `y` (BATCH * N residues, (lo, hi) int64 limb pairs) as
+    ntt_out.npy: DUMP_SAMPLE x 4 float64, the 32-bit limbs of each residue, least significant first (float64
+    holds them exactly), and ntt_out_index.npy: the flat index (transform * N + position) of each row."""
+    import numpy as np
+    import torch
+    idx = np.sort(np.random.default_rng(0).choice(BATCH * N, DUMP_SAMPLE, replace=False))
+    v = y[torch.from_numpy(idx).to(y.device)].cpu().numpy().view(np.uint64)
+    limbs = np.stack([v[:, 0] & 0xFFFFFFFF, v[:, 0] >> 32, v[:, 1] & 0xFFFFFFFF, v[:, 1] >> 32], axis=1)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "ntt_out.npy"), limbs.astype(np.float64))
+    np.save(os.path.join(out_dir, "ntt_out_index.npy"), idx.astype(np.float64))
 
 
 def cpu_arm(steps, warmup, batch):
@@ -346,6 +364,8 @@ def run_ours(args):
     ms = float(t.item())
     ms_per_step = ms / args.steps
     value = world * BATCH * BUTTERFLIES_PER_NTT * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:  # (before the legs below reuse y)
+        dump_outputs(args.dump_outputs, y)
 
     # ---- the chip's measured 128-bit butterfly rate (montmul + add + sub on registers, no memory):
     #      the compute roof this kernel actually lives under (profiles/r01_notes.md)
@@ -617,7 +637,13 @@ def main():
     ap.add_argument("--steps", type=int, default=500)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of rank 0's last step output to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,13 +6,16 @@
     pickle identity) without a GPU;
   * tests/test_dropin_gpu.py  -- engine = the CUDA engine: the parity tests proper.
 """
+import gzip
 import hashlib
+import json
+import os
 import pickle
 import random
 
 import pytest
 
-from conftest import load_golden
+from conftest import GOLDEN, load_golden
 from hostmirror_loader import load_host_types
 
 T = load_host_types()
@@ -267,6 +270,143 @@ def case_faststark_trace_replay():
         assert idx == rec["indices"]
         want = [T.dec_obj(o) for o in rec["pushed"]]
         assert [pickle.dumps(o) for o in ps.objects[before:]] == [pickle.dumps(o) for o in want]
+
+
+# ------------------------------------------ recorded runs of fast_stark.py / fast_rpsss.py
+def canon(x):
+    """the canonical form make_golden.py's Recorder digests (the same rules, on the drop-in's types)"""
+    import sa_devlist
+    if isinstance(x, bytes):
+        return {"b": x.hex()}
+    if isinstance(x, T.FieldElement):
+        return {"f": str(x.value)}
+    if isinstance(x, T.Polynomial):
+        return {"poly": [str(c.value) for c in x.coefficients]}
+    if isinstance(x, bool):
+        return {"bool": x}
+    if isinstance(x, int):
+        return {"i": x}
+    if isinstance(x, tuple):
+        return {"t": [canon(v) for v in x]}
+    if isinstance(x, (list, sa_devlist.DeviceCodeword)):
+        return {"l": [canon(v) for v in x]}
+    raise TypeError(type(x))
+
+
+def canon_digest(x):
+    return hashlib.sha256(json.dumps(canon(x), separators=(",", ":")).encode()).hexdigest()
+
+
+def decode(c):
+    (k, v), = c.items()
+    if k == "b":
+        return bytes.fromhex(v)
+    if k == "f":
+        return T.fe(v)
+    if k == "poly":
+        return T.poly(v)
+    if k in ("i", "bool"):
+        return v
+    if k == "t":
+        return tuple(decode(x) for x in v)
+    if k == "l":
+        return [decode(x) for x in v]
+    raise ValueError(k)
+
+
+class ReplayStream(F.ProofStream):
+    """A proof stream whose Fiat-Shamir challenges are the recorded ones; each is handed out only if the
+    transcript it is drawn from is, digest for digest, the one the reference drew it from."""
+
+    def __init__(self, objects=(), read_index=0):
+        F.ProofStream.__init__(self)
+        self.objects, self.read_index, self.challenges = list(objects), read_index, []
+
+    def _challenge(self, kind, seen):
+        assert self.challenges, "a challenge the reference did not draw"
+        c = self.challenges.pop(0)
+        assert c["kind"] == kind and c["state"] == canon_digest(list(seen)), "transcript differs at a challenge"
+        return bytes.fromhex(c["out"])
+
+    def prover_fiat_shamir(self, num_bytes=32):
+        return self._challenge("prover_fiat_shamir", self.objects)
+
+    def verifier_fiat_shamir(self, num_bytes=32):
+        return self._challenge("verifier_fiat_shamir", self.objects[:self.read_index])
+
+
+def replay_recorded(name):
+    """Replay a run of the unmodified caller recorded by make_golden.py (Recorder): every call it made into the
+    drop-in surface, in order, with the drop-in's own earlier results as the arguments that were results, must
+    give the reference's result (digest), push what the reference pushed and draw the challenges it drew; the
+    caller's own pushes are rebuilt from the drop-in's results.  Returns the recorded file and the streams."""
+    with gzip.open(os.path.join(GOLDEN, name), "rt") as f:
+        g = json.load(f)
+    results, streams = {}, {}  # event index -> the drop-in's result; stream number -> ReplayStream
+
+    def arg(a):
+        if "ref" in a:
+            return results[a["ref"]]
+        if "out" in a:
+            return []
+        if "stream" in a:
+            ps = streams.get(a["stream"])
+            if ps is None:  # a stream the caller filled itself (a deserialized proof): one with the same objects
+                src = [s for s in streams.values() if canon_digest(s.objects) == a["objects"]]
+                assert src, "no replayed stream holds the objects this call was given"
+                ps = streams[a["stream"]] = ReplayStream(src[0].objects)
+            ps.read_index = a["read_index"]
+            assert canon_digest(ps.objects) == a["objects"]
+            return ps
+        return decode(a)
+    for i, ev in enumerate(g["events"]):
+        if "push" in ev:
+            ps = streams.setdefault(ev["push"], ReplayStream())
+            src = ev["obj"]
+            ps.push(results[src["ref"]] if "ref" in src else
+                    results[src["elem"][0]][src["elem"][1]] if "elem" in src else decode(src))
+            continue
+        fn, args = ev["fn"], [arg(a) for a in ev["args"]]
+        where = "event %d (%s)" % (i, fn)
+        stream = next((a for a in args if isinstance(a, ReplayStream)), None)
+        before = len(stream.objects) if stream is not None else 0
+        if stream is not None:
+            stream.challenges = list(ev["fs"])
+        if fn.startswith("fast_"):
+            got = getattr(N, fn)(*args)
+        elif fn.startswith("Merkle."):
+            got = getattr(F.Merkle, fn[7:])(*args)
+        else:
+            off, om, n, ef, tests = ev["fri"]
+            got = getattr(F.Fri(decode(off), decode(om), n, ef, tests), fn[4:])(*args)
+        assert canon_digest(got) == ev["out"], where
+        if stream is not None:
+            assert not stream.challenges, where + ": fewer challenges than the reference drew"
+            assert canon_digest(stream.objects[before:]) == ev["pushed"], where
+        if fn == "Fri.verify":
+            assert canon_digest(args[1]) == ev["out_list"], where
+        results[i] = got
+    return g, streams
+
+
+def case_faststark_proof_replay():
+    """fast_stark.py's seeded prove + verify (tests/golden/faststark_proof.json.gz): the proof assembled from the
+    drop-in's results is the reference's proof, byte for byte, and the verifier's FRI check accepts it"""
+    g, streams = replay_recorded("faststark_proof.json.gz")
+    proof = streams[0].serialize()
+    assert hashlib.sha256(proof).hexdigest() == g["proof_sha256"] and len(proof) == g["proof_len"]
+    verdicts = [e["out"] for e in g["events"] if e.get("fn") == "Fri.verify"]
+    assert g["verify"] is True and verdicts == [canon_digest(True)]
+
+
+def case_rpsss_replay():
+    """fast_rpsss.py's seeded keygen, sign and two verifies (tests/golden/rpsss_run.json.gz): the signature
+    assembled from the drop-in's results is the reference's, byte for byte; every FRI verdict is the reference's"""
+    g, streams = replay_recorded("rpsss_run.json.gz")
+    sig = streams[0].serialize()
+    assert hashlib.sha256(sig).hexdigest() == g["signature_sha256"] == load_golden("rpsss.json")["signature_sha256"]
+    assert len(sig) == g["signature_len"]
+    assert g["verify"] is True and g["verify_other_document"] is False
 
 
 # --------------------------------------------------------------------- merkle

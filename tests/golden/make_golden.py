@@ -1,11 +1,12 @@
 #!/usr/bin/env python3
 """Generate tests/golden/*.json by running the UNMODIFIED Python reference.
 
-Run in the dev container only (needs /root/reference/code; the GPU box has no
-reference).  The fixtures pin both the CPU oracle (tests/test_oracle.py) and the
-CUDA engine (tests/test_*_gpu.py) to the reference's own outputs.
+Needs a checkout of the reference: STARK_REFERENCE names its code/ directory.
+The fixtures pin the CPU oracle (tests/test_oracle.py), the CUDA engine
+(tests/test_*_gpu.py) and the host mirror (tests/test_hostmirror.py) to the
+reference's own outputs, so the tests themselves never need the reference.
 
-    python tests/golden/make_golden.py            # ~2-3 minutes
+    STARK_REFERENCE=<checkout>/code python tests/golden/make_golden.py    # ~2-3 minutes
 
 Encoding: field elements are decimal strings, digests/bytes are hex strings.
 Seeds are stated per case; inputs come from random.Random(seed).randrange(p).
@@ -15,10 +16,13 @@ import json
 import os
 import pickle
 import random
+import subprocess
 import sys
 
 sys.dont_write_bytecode = True
-REF = os.environ.get("STARK_REFERENCE", "/root/reference/code")
+REF = os.environ.get("STARK_REFERENCE")
+if not REF or not os.path.isdir(REF):
+    sys.exit("make_golden.py: set STARK_REFERENCE to the reference checkout's code/ directory")
 sys.path.insert(0, REF)
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -67,6 +71,15 @@ def dump(name, obj):
     path = os.path.join(HERE, name)
     with open(path, "w") as f:
         json.dump(obj, f, separators=(",", ":"))
+    print(f"{name}: {os.path.getsize(path)} bytes")
+
+
+def dump_gz(name, obj):
+    """gzip-compressed JSON (mtime 0, so the same data gives the same bytes)"""
+    import gzip
+    path = os.path.join(HERE, name)
+    with gzip.GzipFile(path, "wb", compresslevel=9, mtime=0) as f:
+        f.write(json.dumps(obj, separators=(",", ":")).encode())
     print(f"{name}: {os.path.getsize(path)} bytes")
 
 
@@ -430,8 +443,217 @@ def gen_rpsss():
         os.urandom = real_urandom
 
 
+# ---------------------------- recorded runs of fast_stark.py / fast_rpsss.py (tests/dropin_cases.py replays them)
+def canon(x):
+    """JSON-able canonical form of a value crossing the drop-in surface (independent of the classes' modules)"""
+    if isinstance(x, bytes):
+        return {"b": x.hex()}
+    if isinstance(x, FieldElement):
+        return {"f": str(x.value)}
+    if isinstance(x, Polynomial):
+        return {"poly": [str(c.value) for c in x.coefficients]}
+    if isinstance(x, bool):
+        return {"bool": x}
+    if isinstance(x, int):
+        return {"i": x}
+    if isinstance(x, tuple):
+        return {"t": [canon(v) for v in x]}
+    if isinstance(x, list):
+        return {"l": [canon(v) for v in x]}
+    raise TypeError(type(x))
+
+
+def canon_digest(x):
+    return hashlib.sha256(json.dumps(canon(x), separators=(",", ":")).encode()).hexdigest()
+
+
+class Recorder:
+    """Records, in order, every top-level call the caller makes into the drop-in surface (the ntt.py functions,
+    Merkle.commit / open, Fri.prove / verify), every object the caller pushes onto a proof stream (as a reference
+    to the call result it came from where it did) and the Fiat-Shamir challenges drawn inside recorded calls
+    together with the transcript state they were drawn from.  Arguments that are earlier results are stored as
+    references, results as canonical digests."""
+
+    def __init__(self):
+        self.events, self.results, self.keep = [], {}, []
+        self.elems, self.streams, self.depth, self.current = {}, {}, 0, None
+
+    def _result(self, k, res):
+        self.keep.append(res)
+        self.results[id(res)] = k
+        if isinstance(res, list):
+            for i, e in enumerate(res):
+                self.elems.setdefault(id(e), (k, i))
+
+    def stream_id(self, ps):
+        self.keep.append(ps)
+        return self.streams.setdefault(id(ps), len(self.streams))
+
+    def arg(self, a):
+        if id(a) in self.results:
+            return {"ref": self.results[id(a)]}
+        if isinstance(a, ProofStream):
+            return {"stream": self.stream_id(ps=a), "objects": canon_digest(list(a.objects)), "read_index": a.read_index}
+        if isinstance(a, list) and not a:
+            return {"out": []}
+        return canon(a)
+
+    def wrap(self, owner, name, label, method=False, static=False):
+        orig = getattr(owner, name)
+        rec = self
+
+        def w(*a):
+            if rec.depth:
+                return orig(*a)
+            args = a[1:] if method else a
+            ev = {"fn": label, "args": [rec.arg(x) for x in args], "fs": []}
+            if method:
+                s = a[0]
+                ev["fri"] = [canon(s.offset), canon(s.omega), s.domain_length, s.expansion_factor, s.num_colinearity_tests]
+            streams = [x for x in args if isinstance(x, ProofStream)]
+            before = len(streams[0].objects) if streams else 0
+            rec.depth, rec.current = 1, ev
+            try:
+                res = orig(*a)
+            finally:
+                rec.depth, rec.current = 0, None
+            ev["out"] = canon_digest(res)
+            if label == "Fri.prove":
+                ev["indices"] = res
+            if streams:
+                ev["pushed"] = canon_digest(list(streams[0].objects[before:]))
+            if label == "Fri.verify":
+                ev["out_list"] = canon_digest(args[1])
+            rec._result(len(rec.events), res)
+            rec.events.append(ev)
+            return res
+        setattr(owner, name, staticmethod(w) if static else w)
+
+    def wrap_push(self, cls):
+        orig = cls.push
+        rec = self
+
+        def push(ps, obj):
+            if not rec.depth:
+                if id(obj) in rec.results:
+                    src = {"ref": rec.results[id(obj)]}
+                elif id(obj) in rec.elems:
+                    src = {"elem": list(rec.elems[id(obj)])}
+                else:
+                    src = canon(obj)
+                rec.events.append({"push": rec.stream_id(ps), "obj": src})
+            return orig(ps, obj)
+        cls.push = push
+
+    def wrap_fiat_shamir(self, cls):
+        rec = self
+        for kind in ("prover_fiat_shamir", "verifier_fiat_shamir"):
+            orig = cls.__dict__.get(kind)
+            if orig is None:
+                continue
+
+            def fs(ps, *a, _orig=orig, _kind=kind):
+                out = _orig(ps, *a)
+                if rec.current is not None:
+                    seen = ps.objects if _kind == "prover_fiat_shamir" else ps.objects[:ps.read_index]
+                    rec.current["fs"].append({"kind": _kind, "state": canon_digest(list(seen)), "out": out.hex()})
+                return out
+            setattr(cls, kind, fs)
+
+
+def record_run(scenario):
+    """run scenario() with the reference's modules instrumented; returns (its result, the recorded events)"""
+    import fast_stark as fs
+    import fri as reffri
+    import merkle as refmerkle
+    rec = Recorder()
+    ntt_fns = [n for n in dir(fs) if n.startswith("fast_") and callable(getattr(fs, n))]
+    classes = [ProofStream] + ProofStream.__subclasses__()
+    saved = [(fs, n, getattr(fs, n)) for n in ntt_fns]
+    saved += [(refmerkle.Merkle, n, refmerkle.Merkle.__dict__[n]) for n in ("commit", "open")]
+    saved += [(reffri.Fri, n, reffri.Fri.__dict__[n]) for n in ("prove", "verify")]
+    saved += [(c, n, c.__dict__[n]) for c in classes for n in ("push", "prover_fiat_shamir", "verifier_fiat_shamir")
+              if n in c.__dict__]
+    for n in ntt_fns:
+        rec.wrap(fs, n, n)
+    rec.wrap(refmerkle.Merkle, "commit", "Merkle.commit", static=True)
+    rec.wrap(refmerkle.Merkle, "open", "Merkle.open", static=True)
+    rec.wrap(reffri.Fri, "prove", "Fri.prove", method=True)
+    rec.wrap(reffri.Fri, "verify", "Fri.verify", method=True)
+    rec.wrap_push(ProofStream)
+    for c in classes:
+        rec.wrap_fiat_shamir(c)
+    try:
+        return scenario(rec), rec.events
+    finally:
+        for owner, n, f in saved:
+            setattr(owner, n, f)
+
+
+def seeded_urandom(seed):
+    rng = random.Random(seed)
+    return rng, (lambda n: bytes(rng.getrandbits(8) for _ in range(n)))
+
+
+def gen_faststark_proof():
+    """one seeded FastStark.prove + verify (test_fast_stark.py parameters, os.urandom seeded with 600, as in
+    gen_faststark_trace) recorded for tests/dropin_cases.case_faststark_proof_replay"""
+    import fast_stark as fs
+    from rescue_prime import RescuePrime
+    real_urandom = os.urandom
+    rng, os.urandom = seeded_urandom(600)
+
+    def scenario(rec):
+        rp = RescuePrime()
+        stark = fs.FastStark(field, 4, 2, 2, rp.m, rp.N + 1, transition_constraints_degree=3)
+        tz, tzc, tzr = stark.preprocess()
+        x = fe(rng.randrange(P))
+        air = rp.transition_constraints(stark.omicron)
+        boundary = rp.boundary_constraints(rp.hash(x))
+        proof = stark.prove(rp.trace(x), air, boundary, tz, tzc)
+        return proof, stark.verify(proof, air, boundary, tzr)
+    try:
+        (proof, ok), events = record_run(scenario)
+    finally:
+        os.urandom = real_urandom
+    assert ok
+    dump_gz("faststark_proof.json.gz", {"urandom_seed": 600, "events": events, "verify": ok,
+                                  "proof_sha256": hashlib.sha256(proof).hexdigest(), "proof_len": len(proof)})
+
+
+def gen_rpsss_run():
+    """FastRPSSS keygen, sign(b"Hello, World!"), verify of that document and of b"Byebye." (os.urandom seeded
+    with 700, as in gen_rpsss), recorded for tests/dropin_cases.case_rpsss_replay.  ~8 minutes."""
+    import fast_rpsss
+    real_urandom = os.urandom
+    rng, os.urandom = seeded_urandom(700)
+
+    def scenario(rec):
+        r = fast_rpsss.FastRPSSS()
+        sk, pk = r.keygen()
+        sig = r.sign(sk, b"Hello, World!")
+        return sig, r.verify(pk, b"Hello, World!", sig), r.verify(pk, b"Byebye.", sig)
+    try:
+        (sig, good, bad), events = record_run(scenario)
+    finally:
+        os.urandom = real_urandom
+    assert good and not bad
+    dump_gz("rpsss_run.json.gz", {"urandom_seed": 700, "events": events, "verify": good, "verify_other_document": bad,
+                            "signature_sha256": hashlib.sha256(sig).hexdigest(), "signature_len": len(sig)})
+
+
+# ------------------------------------------- value types, as tests/test_hostmirror.py exercises them
+def gen_hostmirror():
+    """sha256 and length of the text tests/test_hostmirror.py's SCRIPT prints with the reference's own
+    algebra / univariate / merkle / ip modules; the mirror in stark-anatomy_b200/hostmirror must print the same"""
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_hostmirror import SCRIPT
+    out = subprocess.check_output([sys.executable, "-c", SCRIPT, REF], text=True)
+    dump("hostmirror.json", {"sha256": hashlib.sha256(out.encode()).hexdigest(), "len": len(out)})
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["field", "ntt", "poly", "merkle", "fri", "faststark"]
+    which = sys.argv[1:] or ["field", "ntt", "poly", "merkle", "fri", "faststark", "hostmirror", "faststark_proof"]
     if "field" in which:
         gen_field()
     if "ntt" in which:
@@ -444,6 +666,12 @@ if __name__ == "__main__":
         gen_fri()
     if "faststark" in which:
         gen_faststark_trace()
+    if "hostmirror" in which:
+        gen_hostmirror()
+    if "faststark_proof" in which:
+        gen_faststark_proof()
+    if "rpsss_run" in which:  # not in the default set: ~8 min
+        gen_rpsss_run()
     if "fri20" in which:      # not in the default set: ~75 s
         gen_fri_2_20()
     if "rpsss" in which:      # not in the default set: ~40 s

@@ -1,9 +1,10 @@
 """Test helper: load the host value types the drop-in modules will use.
 
-``load_host_types()`` puts stark-anatomy_b200/ (and, when present, the reference's
-code/ directory behind it) on sys.path exactly like a user of the drop-in would,
-imports the drop-in ``ntt`` / ``fri`` modules and returns a small namespace with
-the value types plus JSON fixture decoders.
+``load_host_types()`` puts stark-anatomy_b200/ (and, when STARK_REFERENCE names a
+checkout of the reference's code/ directory, that directory behind it) on sys.path
+exactly like a user of the drop-in would, imports the drop-in ``ntt`` / ``fri``
+modules and returns a small namespace with the value types plus JSON fixture decoders.
+Without STARK_REFERENCE the drop-in uses its own host mirror of the value types.
 """
 import importlib
 import os
@@ -13,25 +14,15 @@ import types
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "stark-anatomy_b200")
 
-
-
-def _find_reference():
-    """the reference's flat module directory: the read-only checkout in the dev container, else the copy
-    staged by __graft_entry__.stage_reference() under the git-ignored baseline/_ref/ (which travels to the
-    GPU box with the gpurun snapshot)"""
-    for cand in (os.environ.get("STARK_REFERENCE"), "/root/reference/code", os.path.join(ROOT, "baseline", "_ref", "code")):
-        if cand and os.path.isdir(cand):
-            return cand
-    return "/root/reference/code"
-
-
-REFERENCE = _find_reference()
+# the reference's flat module directory; also enables the tests that run its modules unmodified
+REFERENCE = os.environ.get("STARK_REFERENCE", "")
+HAVE_REFERENCE = bool(REFERENCE) and os.path.isdir(REFERENCE)
 
 
 def setup_paths(use_reference=True):
     """drop-in first, then (optionally) the reference's flat module directory"""
     sys.dont_write_bytecode = True
-    if use_reference and os.path.isdir(REFERENCE) and REFERENCE not in sys.path:
+    if use_reference and HAVE_REFERENCE and REFERENCE not in sys.path:
         sys.path.insert(0, REFERENCE)
     if PKG in sys.path:
         sys.path.remove(PKG)

@@ -13,15 +13,27 @@ import dropin_cases as C
 import sa_engine
 from fake_engine import OracleEngine
 from conftest import load_golden, ROOT
-from hostmirror_loader import REFERENCE
+from hostmirror_loader import HAVE_REFERENCE, REFERENCE
+
+# these run the reference's own modules unmodified on top of the drop-in, so they need a checkout of it
+needs_reference = pytest.mark.skipif(not HAVE_REFERENCE, reason="STARK_REFERENCE does not name the reference's code/ directory")
+
+
+def drop_cached_trees():
+    """fri.Merkle caches device trees by data fingerprint, and a tree belongs to the engine that built it:
+    none may cross an engine swap (the GPU tests commit the same golden data on the CUDA engine)"""
+    C.F.Merkle._trees.clear()
+    C.F.Merkle._cache_bytes = 0
 
 
 @pytest.fixture(autouse=True)
 def double_engine():
     prev = sa_engine._ENGINE
+    drop_cached_trees()
     sa_engine.set_engine(OracleEngine())
     yield
     sa_engine.set_engine(prev)
+    drop_cached_trees()
 
 
 def test_ntt_vectors():
@@ -96,11 +108,16 @@ def test_default_engine_fails_loudly_without_cuda():
         C.N.ntt(C.T.field.primitive_nth_root(16), C.seeded(1, 16))
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present")
 def test_unmodified_fast_stark_prove_is_byte_identical():
-    """code/fast_stark.py, UNMODIFIED, imported with the drop-in ahead of it on sys.path:
-    with os.urandom seeded as in tests/golden/make_golden.py the proof must be the same
-    bytes the pure reference produced, and the reference verifier must accept it."""
+    """code/fast_stark.py, UNMODIFIED, with the drop-in ahead of it on sys.path and os.urandom seeded as in
+    tests/golden/make_golden.py: the proof must be the same bytes the pure reference produced, and the
+    reference verifier must accept it.  Every call fast_stark.py made into the drop-in during that prove and
+    verify is recorded in tests/golden/faststark_proof.json.gz; replaying them rebuilds the proof from the
+    drop-in's results.  With STARK_REFERENCE set, fast_stark.py itself runs on the drop-in as well."""
+    C.case_faststark_proof_replay()
+    assert len(sa_engine.get_engine().calls) > 10
+    if not HAVE_REFERENCE:
+        return
     code = r'''
 import sys, os, random, hashlib
 sys.dont_write_bytecode = True
@@ -139,7 +156,7 @@ print(hashlib.sha256(proof).hexdigest(), len(proof), ok, len(sa_engine.get_engin
     assert out2[:3] == out[:3] and int(out2[3]) > int(out[3])
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present")
+@needs_reference
 @pytest.mark.parametrize("ref_test", ["test_ntt.py", "test_fri.py", "test_merkle.py"])
 def test_reference_own_tests_pass_against_the_dropin(ref_test):
     """The reference's OWN test files (code/test_ntt.py, test_fri.py, test_merkle.py), unmodified,
@@ -156,8 +173,9 @@ sa_engine.set_engine(OracleEngine())
 import ntt, fri
 assert ntt.__file__.startswith(%(pkg)r) and fri.__file__.startswith(%(pkg)r)
 import pytest
+# (--confcutdir: collection does not walk the directories above the reference, which may not be listable)
 rc = pytest.main([%(target)r, "-q", "-x", "-k", "not colinearity", "-p", "no:cacheprovider",
-                  "--rootdir", %(ref)r, "-c", "/dev/null", "--import-mode=importlib"])
+                  "--rootdir", %(ref)r, "--confcutdir", %(ref)r, "-c", "/dev/null", "--import-mode=importlib"])
 eng = sa_engine.get_engine()
 print("RC", int(rc), "ENGINE_CALLS", len(eng.calls))
 ''' % {"pkg": os.path.join(ROOT, "stark-anatomy_b200"), "ref": REFERENCE,
@@ -171,11 +189,17 @@ print("RC", int(rc), "ENGINE_CALLS", len(eng.calls))
         assert int(tail[3]) > 0, "the reference test did not reach the engine"
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present")
 def test_unmodified_fast_rpsss_sign_and_verify():
     """BASELINE config 5's functional check: code/fast_rpsss.py and code/fast_stark.py, unmodified, on top
-    of the drop-in (with the opt-in device Polynomial.__mul__): keygen -> sign -> verify is True, and a
-    signature does not verify for another document.  (Reference alone: sign 29 s, verify 206 s.)"""
+    of the drop-in: keygen -> sign -> verify is True, and a signature does not verify for another document.
+    (Reference alone: sign 29 s, verify 206 s.)  The calls they made into the drop-in during a seeded run are
+    recorded in tests/golden/rpsss_run.json.gz; replaying them rebuilds the signature from the drop-in's results.
+    With STARK_REFERENCE set, the two modules themselves run on the drop-in as well (with the opt-in device
+    Polynomial.__mul__)."""
+    C.case_rpsss_replay()
+    assert len(sa_engine.get_engine().calls) > 50
+    if not HAVE_REFERENCE:
+        return
     code = r'''
 import sys
 sys.dont_write_bytecode = True

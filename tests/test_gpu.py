@@ -772,6 +772,13 @@ def test_dropin_faststark_trace_replay(eng):
     C.case_faststark_trace_replay()
 
 
+def test_dropin_recorded_faststark_and_rpsss_runs(eng):
+    """the recorded calls of fast_stark.py's prove + verify and of fast_rpsss.py's keygen / sign / verify,
+    replayed on the CUDA engine: the same proof and signature bytes as the pure reference"""
+    C.case_faststark_proof_replay()
+    C.case_rpsss_replay()
+
+
 def test_dropin_merkle_class(eng):
     C.case_merkle_class()
 
@@ -785,9 +792,9 @@ def test_dropin_device_list(eng):
 
 
 def test_config5_unmodified_faststark_and_rpsss_on_the_cuda_engine(eng):
-    """BASELINE config 5 on the real engine: the reference's fast_stark.py / fast_rpsss.py, unmodified (staged
-    under baseline/_ref/code by __graft_entry__.stage_reference; /root/reference does not exist on the GPU
-    box), on top of the drop-in.  The seeded proof and the seeded signature must be the bytes the pure
+    """BASELINE config 5 on the real engine: the reference's fast_stark.py / fast_rpsss.py, unmodified (from
+    the checkout whose code/ directory STARK_REFERENCE names; skipped without one), on top of the
+    drop-in.  The seeded proof and the seeded signature must be the bytes the pure
     reference produced (tests/golden/faststark_trace.json, rpsss.json) and must verify; between
     fast_coset_evaluate and Fri.prove no 2^k-element list may cross the PCIe link (section 8 f3)."""
     import json

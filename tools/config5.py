@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """BASELINE config 5 on the real CUDA engine: the reference's code/fast_stark.py and code/fast_rpsss.py,
-UNMODIFIED (imported from the staged copy under baseline/_ref/code or from /root/reference/code), with the
+UNMODIFIED (imported from the checkout of the reference whose code/ directory STARK_REFERENCE names), with the
 drop-in ntt.py / fri.py ahead of them on sys.path and the default engine (CUDA, no test double).
 
     python tools/config5.py [--out gpurun_out/r02_config5.json] [--skip-rpsss]
@@ -24,10 +24,8 @@ PKG = os.path.join(ROOT, "stark-anatomy_b200")
 
 
 def find_reference():
-    for cand in (os.environ.get("STARK_REFERENCE"), "/root/reference/code", os.path.join(ROOT, "baseline", "_ref", "code")):
-        if cand and os.path.isdir(cand):
-            return cand
-    return None
+    cand = os.environ.get("STARK_REFERENCE")
+    return cand if cand and os.path.isdir(cand) else None
 
 
 COMMON = r'''
@@ -112,7 +110,7 @@ def main():
     args = ap.parse_args()
     ref = find_reference()
     if ref is None:
-        print(json.dumps({"unavailable": "no reference checkout (/root/reference/code or baseline/_ref/code)"}))
+        print(json.dumps({"unavailable": "STARK_REFERENCE does not name the reference's code/ directory"}))
         return 0
     fmt = {"pkg": PKG, "ref": ref}
     golden = os.path.join(ROOT, "tests", "golden")

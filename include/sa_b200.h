@@ -185,15 +185,6 @@ int sa_fri_commit(void *layers, void *trees, const void *codeword, size_t n, int
                   const uint64_t offset[2], const uint64_t omega[2], sa_fri_challenge_fn challenge, void *user,
                   void *stream);
 
-/* How sa_fri_commit runs the narrow rounds (<= 2^16 leaves): 0 = one launch per round (the default); 1 = ONE
- * persistent launch for all of them (SA_FRI_PERSISTENT=1) - the kernel publishes each root into mapped host memory
- * and waits there for the challenge - provided the start-up probe found that the host can reach a running kernel
- * (ncu, compute-sanitizer and CUDA_LAUNCH_BLOCKING serialise launches: then it stays 0); -1 = not decided yet (no
- * commit has run).  Results are identical; measured on B200 the two are equally fast (the narrow rounds are
- * blake2b dependency chains, not launch overhead), so the simpler one is the default.  A tail kernel that does not
- * get its challenge within SA_FRI_TAIL_TIMEOUT_S (default 20) seconds gives up and the commit returns SA_ECUDA. */
-int sa_fri_tail_mode(void);
-
 /* ---- device memory the library keeps between calls (no reference counterpart) ------------------
  * Twiddle tables (per device, log n, root, direction) and FRI x^-1 tables (per device, omega, n)
  * live in one least-recently-used cache bounded by bytes: default 4 GiB, SA_CACHE_LIMIT_MIB, or

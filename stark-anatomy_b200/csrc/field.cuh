@@ -189,28 +189,15 @@ __device__ __forceinline__ fe fe_cond_sub_p(uint32_t r0, uint32_t r1, uint32_t r
     return fe_make(use ? d0 : r0, use ? d1 : r1, use ? d2 : r2, use ? d3 : r3);
 }
 // (d3..d0) + p when m is all-ones, unchanged when m is zero (m = the borrow word of a subtraction that
-// went negative).  The two mask words (1 and P3, or zeros) are either ANDs (ALU pipe) or products of the
-// all-ones word (FMA pipe).  SA_FIELD_MASK says which are ANDs: bit 0 = montmul's w, bit 1 = montmul's
-// add-back, bit 2 = fe_sub's add-back.  Measured on the 16 x 2^20 NTT step (profiles/r01g_field_v2.txt):
-// 1 -> 0.737 ms, 0 -> 0.741, 4 -> 0.748, 7 -> 0.758.
-#ifndef SA_FIELD_MASK
-#define SA_FIELD_MASK 1
-#endif
-// SA_MONTMUL_V: 1 = multiply-accumulate chain reduction (round 1), 2 = even/odd reduction (see fe_montmul)
-#ifndef SA_MONTMUL_V
-#define SA_MONTMUL_V 1
-#endif
-template <bool ALU_MASKS>
+// went negative).  The two mask words (1 and P3, or zeros) are products of the all-ones word, so they
+// issue on the FMA pipe rather than the ALU pipe.  Measured on the 16 x 2^20 NTT step
+// (profiles/r01g_field_v2.txt): montmul's w an AND and both add-backs multiplies (the form used here)
+// 0.737 ms; all three multiplies 0.741; only fe_sub's add-back an AND 0.748; all three ANDs 0.758.
 __device__ __forceinline__ fe fe_cond_add_p(uint32_t d0, uint32_t d1, uint32_t d2, uint32_t d3, uint32_t m) {
     uint32_t p0, p3;
-    if (ALU_MASKS) {
-        p0 = m & 1u;
-        p3 = m & 0xCB800000u;
-    } else {
-        asm("mul.lo.u32 %0, %2, %2;\n\t"           // (-1)^2 = 1
-            "mul.lo.u32 %1, %2, 0x34800000;"        // (-1) * (-P3) = P3
-            : "=r"(p0), "=r"(p3) : "r"(m));
-    }
+    asm("mul.lo.u32 %0, %2, %2;\n\t"           // (-1)^2 = 1
+        "mul.lo.u32 %1, %2, 0x34800000;"        // (-1) * (-P3) = P3
+        : "=r"(p0), "=r"(p3) : "r"(m));
     uint32_t r0, r1, r2, r3;
     asm("add.cc.u32 %0, %4, %8;\n\t"
         "addc.cc.u32 %1, %5, 0;\n\t"
@@ -245,7 +232,7 @@ __device__ __forceinline__ fe fe_sub(const fe &a, const fe &b) {
         : "=r"(d0), "=r"(d1), "=r"(d2), "=r"(d3), "=r"(m)
         : "r"(a.v[0]), "r"(a.v[1]), "r"(a.v[2]), "r"(a.v[3]), "r"(b.v[0]), "r"(b.v[1]), "r"(b.v[2]),
           "r"(b.v[3]));
-    return fe_cond_add_p<((SA_FIELD_MASK) >> 2) & 1>(d0, d1, d2, d3, m);
+    return fe_cond_add_p(d0, d1, d2, d3, m);
 }
 __device__ __forceinline__ fe fe_montmul(const fe &a, const fe &b) {
     uint32_t a0 = a.v[0], a1 = a.v[1], a2 = a.v[2], a3 = a.v[3];
@@ -300,69 +287,19 @@ __device__ __forceinline__ fe fe_montmul(const fe &a, const fe &b) {
           "=&r"(o0), "=&r"(o1), "=&r"(o2), "=&r"(o3), "=&r"(o4), "=&r"(o5), "=&r"(o6)
         : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1), "r"(b2), "r"(b3));
     (void)o0; (void)o1; (void)o2; (void)o3; (void)o4; (void)o5; (void)o6;
-#if SA_MONTMUL_V >= 2
-    // Reduction, even/odd form.  m = t_lo * p^-1 mod 2^128 = (e0, e1, e2, e3 - x) with x = e0*P3 mod 2^32 and
-    // w = the borrow of that top word; t * 2^-128 = t_hi - ((m*P3) >> 32) - w.  The four products m_i*P3 are
-    // taken as independent 64-bit values: E = m0*P3 + (m2*P3 << 64), O = m1*P3 + (m3*P3 << 64), so
-    // m*P3 = E + (O << 32) and  t_hi - ((m*P3) >> 32) - w = t_hi - (E1, E2, E3, 0) - (O0|w, O1, O2, O3):
-    // two borrow chains on the ALU pipe instead of a multiply-accumulate chain whose 64-bit addends have
-    // to be assembled with register moves (which ptxas issues on the FMA pipe, the one that is short).
-    // O0 = lo(m1*P3) has 23 zero low bits, so OR-ing the borrow bit w into it is the same as adding it.
-    {
-        uint32_t x = e0 * P3;
-        uint32_t m3, nw;
-        asm("sub.cc.u32 %0, %2, %3;\n\t"
-            "subc.u32 %1, 0, 0;"
-            : "=r"(m3), "=r"(nw)
-            : "r"(e3), "r"(x));
-        uint32_t E0, E1, E2, E3, O0, O1, O2, O3;
-        asm("mul.lo.u32 %0, %8, 0xCB800000;\n\t"
-            "mul.hi.u32 %1, %8, 0xCB800000;\n\t"
-            "mul.lo.u32 %2, %10, 0xCB800000;\n\t"
-            "mul.hi.u32 %3, %10, 0xCB800000;\n\t"
-            "mul.lo.u32 %4, %9, 0xCB800000;\n\t"
-            "mul.hi.u32 %5, %9, 0xCB800000;\n\t"
-            "mul.lo.u32 %6, %11, 0xCB800000;\n\t"
-            "mul.hi.u32 %7, %11, 0xCB800000;"
-            : "=r"(E0), "=r"(E1), "=r"(E2), "=r"(E3), "=r"(O0), "=r"(O1), "=r"(O2), "=r"(O3)
-            : "r"(e0), "r"(e1), "r"(e2), "r"(m3));
-        (void)E0;
-        O0 |= nw & 1u;
-        uint32_t r0, r1, r2, r3, ta, tb;
-        asm("sub.cc.u32 %0, %5, %9;\n\t"
-            "subc.cc.u32 %1, %6, %10;\n\t"
-            "subc.cc.u32 %2, %7, %11;\n\t"
-            "subc.cc.u32 %3, %8, 0;\n\t"
-            "subc.u32 %4, 0, 0;"
-            : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3), "=r"(ta)
-            : "r"(e4), "r"(e5), "r"(e6), "r"(e7), "r"(E1), "r"(E2), "r"(E3));
-        asm("sub.cc.u32 %0, %0, %5;\n\t"
-            "subc.cc.u32 %1, %1, %6;\n\t"
-            "subc.cc.u32 %2, %2, %7;\n\t"
-            "subc.cc.u32 %3, %3, %8;\n\t"
-            "subc.u32 %4, 0, 0;"
-            : "+r"(r0), "+r"(r1), "+r"(r2), "+r"(r3), "=r"(tb)
-            : "r"(O0), "r"(O1), "r"(O2), "r"(O3));
-        // the true value lies in (-p, p): at most one of the two chains wrapped
-        return fe_cond_add_p<true>(r0, r1, r2, r3, ta | tb);
-    }
-#endif
     // Reduction with p^-1 = 1 - P3*2^96 (mod 2^128) instead of -p^-1: m = t_lo * p^-1 mod 2^128 is t_lo
     // with (t0*P3 mod 2^32) taken off its top word, and since t_lo - m and m*P3*2^96 cancel below bit
     // 128,  t*2^-128 = t_hi - ((m*P3) >> 32) - w  (w = the borrow of that top word), in (-p, p): one
     // masked add of p.  Half the ALU instructions of the m = -t_lo form (no 128-bit negation, no
-    // five-way select); the 0/1 words come from multiplies so that they issue on the FMA pipe.
+    // five-way select); the add-back's mask words come from multiplies so that they issue on the FMA
+    // pipe, while w is an AND (the fastest split, see fe_cond_add_p).
     uint32_t x = e0 * P3;
     uint32_t m3, nw;
     asm("sub.cc.u32 %0, %2, %3;\n\t"
         "subc.u32 %1, 0, 0;"
         : "=r"(m3), "=r"(nw)
         : "r"(e3), "r"(x));
-    uint32_t w;
-    if ((SA_FIELD_MASK) & 1)
-        w = nw & 1u;
-    else
-        asm("mul.lo.u32 %0, %1, %1;" : "=r"(w) : "r"(nw));  // nw is 0 or -1
+    const uint32_t w = nw & 1u;
     uint32_t u1, u2, u3, u4;
     asm("mad.hi.u32 %0, %4, 0xCB800000, %8;\n\t"
         "mad.lo.cc.u32 %0, %5, 0xCB800000, %0;\n\t"
@@ -381,7 +318,7 @@ __device__ __forceinline__ fe fe_montmul(const fe &a, const fe &b) {
         "subc.u32 %4, 0, 0;"
         : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3), "=r"(top)
         : "r"(e4), "r"(e5), "r"(e6), "r"(e7), "r"(u1), "r"(u2), "r"(u3), "r"(u4));
-    return fe_cond_add_p<((SA_FIELD_MASK) >> 1) & 1>(r0, r1, r2, r3, top);
+    return fe_cond_add_p(r0, r1, r2, r3, top);
 }
 #else
 SA_HD fe fe_add(const fe &a, const fe &b) { return fe_add_portable(a, b); }

@@ -103,8 +103,7 @@ SA_HD void merkle_bottom(uint64_t d[8], const MerkleArgs &a, long long g) {
         v = a.values[g];
     } else {
         const fe t_m = fe_montmul(a.xinv[g], a.s_m);
-        // (.cg: in the persistent tail kernel the previous layer was written by other CTAs of the SAME launch;
-        //  the layer is read exactly once anyway, so bypassing L1 costs nothing elsewhere)
+        // (.cg: each element of the previous layer is read exactly once, so there is nothing to cache in L1)
         v = fri_fold_one(merkle_ld_stream(a.prev + g), merkle_ld_stream(a.prev + a.width + g), t_m, a.inv2_m);
         a.next[g] = v;
     }
@@ -136,31 +135,5 @@ SA_HD void merkle_private(uint64_t root[8], const MerkleArgs &a, long long blk, 
     }
     for (int i = 0; i < 8; i++) root[i] = d[i];
 }
-
-// ---- persistent tail of Fri.commit: the rounds of <= FRI_TAIL_MAX_WIDTH leaves in ONE launch ----
-// Those rounds are blake2b dependency chains of ~1.2 us per tree level; launching a kernel per round and
-// handing its root to the host through a stream added ~20 us to each.  The tail kernel keeps its CTAs
-// resident across rounds: the last CTA of a round publishes the root into mapped host memory, the host
-// answers with the Fiat-Shamir challenge through the same page, CTA 0 forwards it through a device flag.
-constexpr int FRI_TAIL_MAX_ROUNDS = 16;
-constexpr int FRI_TAIL_MAX_LOG = 16;      // widest round handled in the tail: 2^16 leaves (128 CTAs)
-constexpr int FRI_TAIL_MAX_CTAS = 128;    // all of them must be co-resident (296 slots on B200)
-struct FriTailArgs {
-    int nrounds;                 // rounds handled by this launch
-    long long width0;            // leaves of the first tail round (= length of its folded codeword)
-    const fe *prev0;             // the codeword the first tail round folds (2 * width0 elements)
-    fe *layer[FRI_TAIL_MAX_ROUNDS];          // folded codeword of tail round i (width0 >> i elements)
-    uint64_t *tree[FRI_TAIL_MAX_ROUNDS];     // its tree (2 * (width0 >> i) nodes)
-    const fe *xinv[FRI_TAIL_MAX_ROUNDS];     // omega_i^-j tables
-    fe inv2_m;
-    fe s_m0;                     // alpha * 2^-1 * offset^-1 of the first tail round (the host has that challenge)
-    unsigned int *ticket;        // CTA arrival counter of the tree reduction (zero between rounds)
-    unsigned long long *bcast;   // device: [0] = sequence of the newest forwarded challenge, [2..3] = its s_m limbs
-    volatile uint64_t *host;     // mapped page: [0..7] root, [8] root sequence, [16..17] s_m, [18] s_m sequence,
-                                 //              [19] abort request (host), [20] error report (device)
-    unsigned long long seq0;     // tail round i publishes its root with sequence seq0 + i and, for i >= 1,
-                                 // waits for the challenge with sequence seq0 + i - 1
-    long long spin_limit;        // clock64 ticks after which a wait gives up (error report, kernel exits)
-};
 
 }  // namespace sa

@@ -311,77 +311,6 @@ __global__ void __launch_bounds__(256) k_push_mcast(fe *mc, const fe *src, size_
     for (; i < n16; i += stride) tile_st_multicast(mc + i, tile_ld(src + i));
 }
 
-// variant: every CTA streams to ONE destination (CTA c: peer c % ndst, slice c / ndst of the block), so a link sees
-// sequential 512-byte bursts from an SM instead of every SM rotating over all peers (SA_PUSH_MODE=1)
-__global__ void __launch_bounds__(256) k_push_per_peer(const __grid_constant__ PushArgs a, const uint4 *src, size_t n16) {
-    const int peer = blockIdx.x % a.ndst;
-    const size_t part = blockIdx.x / a.ndst, nparts = gridDim.x / a.ndst;
-    uint4 *dst = a.dst[0];
-#pragma unroll
-    for (int p = 1; p < TILE_MAX_PEERS; p++)
-        if (p == peer) dst = a.dst[p];
-    const size_t stride = nparts * blockDim.x;
-    size_t i = part * blockDim.x + threadIdx.x;
-    for (; i + 3 * stride < n16; i += 4 * stride) {
-        uint4 v[4];
-#pragma unroll
-        for (int u = 0; u < 4; u++) v[u] = __ldcs(src + i + u * stride);
-#pragma unroll
-        for (int u = 0; u < 4; u++) dst[i + u * stride] = v[u];
-    }
-    for (; i < n16; i += stride) dst[i] = __ldcs(src + i);
-}
-
-// variant: the TMA engine moves the data (SA_PUSH_MODE=2).  One thread per CTA: bulk-async load of a 16 KB chunk
-// into shared memory (mbarrier), then one bulk-async STORE of the chunk per destination (cp.async.bulk shared ->
-// global, bulk groups); two buffers, so the stores of chunk i drain while chunk i + 1 loads.  Costs the SMs a few
-// instructions per 16 KB and destination, which leaves their issue slots to the transform that runs beside it.
-constexpr uint32_t PUSH_TMA_CHUNK = 16384;
-__global__ void __launch_bounds__(32) k_push_tma(const __grid_constant__ PushArgs a, const char *src, size_t bytes) {
-    __shared__ __align__(128) unsigned char buf[2][PUSH_TMA_CHUNK];
-    __shared__ __align__(8) uint64_t bar[2];
-    if (threadIdx.x != 0) return;
-    const uint32_t bar_a[2] = {(uint32_t)__cvta_generic_to_shared(&bar[0]), (uint32_t)__cvta_generic_to_shared(&bar[1])};
-    const uint32_t buf_a[2] = {(uint32_t)__cvta_generic_to_shared(&buf[0][0]), (uint32_t)__cvta_generic_to_shared(&buf[1][0])};
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a[0]));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a[1]));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    const size_t nchunks = (bytes + PUSH_TMA_CHUNK - 1) / PUSH_TMA_CHUNK;
-    uint32_t phase[2] = {0, 0};
-    int it = 0;
-    for (size_t c = blockIdx.x; c < nchunks; c += gridDim.x, it++) {
-        const int sl = it & 1;
-        const size_t off = c * PUSH_TMA_CHUNK;
-        const uint32_t sz = (uint32_t)((bytes - off) < PUSH_TMA_CHUNK ? (bytes - off) : PUSH_TMA_CHUNK);
-        // the stores issued two chunks ago read this buffer: all but the newest group must be done reading
-        asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a[sl]), "r"(sz) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(buf_a[sl]),
-                     "l"(src + off), "r"(sz), "r"(bar_a[sl])
-                     : "memory");
-        asm volatile(
-            "{\n\t"
-            ".reg .pred p;\n\t"
-            "PUSH_WAIT_%=:\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-            "@p bra PUSH_DONE_%=;\n\t"
-            "bra PUSH_WAIT_%=;\n\t"
-            "PUSH_DONE_%=:\n\t"
-            "}" ::"r"(bar_a[sl]),
-            "r"(phase[sl])
-            : "memory");
-        phase[sl] ^= 1u;
-#pragma unroll
-        for (int p = 0; p < TILE_MAX_PEERS; p++)
-            if (p < a.ndst)
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"((char *)a.dst[p] + off),
-                             "r"(buf_a[sl]), "r"(sz)
-                             : "memory");
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-}
-
 // ---- subproduct tree over a domain of k points (fast_zerofier / fast_interpolate, ntt.py:66-130) ----
 // The k points sit in the first k of K = 2^ceil(log2 k) leaf slots.  Level j has K >> j nodes of
 // m = 2^j coefficients each, stored back to back.  A node whose leaf range lies completely inside the
@@ -557,9 +486,9 @@ __device__ __forceinline__ void merkle_publish_root(const MerkleArgs &a, const u
     out[8] = a.root_seq;
 }
 // the work of one CTA (`blk` of `nblocks`) on one level-range of one tree; sm = MK_THREADS * 8 words of
-// shared memory.  Called once per launch by k_merkle_chunk and once per round by k_fri_tail.
+// shared memory, s_last = one shared word
 __device__ __forceinline__ void merkle_chunk_body(const MerkleArgs &a, const long long blk, const unsigned nblocks,
-                                                  uint64_t *sm) {
+                                                  uint64_t *sm, int &s_last) {
     const int tid = threadIdx.x;
     const int active = a.chunk >> a.ipt_log;  // threads with a private subtree
     uint64_t d[8];
@@ -611,7 +540,6 @@ __device__ __forceinline__ void merkle_chunk_body(const MerkleArgs &a, const lon
         // Every CTA has reduced its chunk to one digest (heap node nblocks + blk).  The CTA that
         // arrives last reduces those nblocks digests as well instead of leaving them to one more
         // launch (each thread fences its own stores, the barrier orders them before the ticket).
-        __shared__ int s_last;
         __threadfence();
         __syncthreads();
         if (tid == 0) s_last = atomicAdd(a.ticket, 1u) == nblocks - 1;
@@ -634,94 +562,12 @@ __device__ __forceinline__ void merkle_chunk_body(const MerkleArgs &a, const lon
     if (a.root_out && tid == 0) merkle_publish_root(a, sm);
 }
 
-// SA_MK_MINB: minimum resident CTAs per SM the register allocator has to leave room for.  2 = at most 128
-// registers: without the bound the kernel drifted to 148 registers in round 2 (one CTA per SM, 2^20-leaf tree
-// 341 -> 383 us); 3 (<= 85 registers, 24 warps per SM) is an experiment
-#ifndef SA_MK_MINB
-#define SA_MK_MINB 2
-#endif
-__global__ void __launch_bounds__(MK_THREADS, SA_MK_MINB) k_merkle_chunk(const __grid_constant__ MerkleArgs a) {
+// At least 2 resident CTAs per SM, so at most 128 registers: without the bound the kernel drifted to 148
+// registers in round 2 (one CTA per SM, 2^20-leaf tree 341 -> 383 us)
+__global__ void __launch_bounds__(MK_THREADS, 2) k_merkle_chunk(const __grid_constant__ MerkleArgs a) {
     __shared__ uint64_t sm[MK_THREADS * 8];
-    merkle_chunk_body(a, blockIdx.x, gridDim.x, sm);
-}
-
-// Persistent tail of Fri.commit (FriTailArgs, fri_merkle.cuh): every round is the fused fold + leaf hash +
-// tree of k_merkle_chunk mode 2 with the last-CTA top reduction; between rounds the CTAs that still have
-// work wait for the next challenge.  Grid = the CTAs of the first (widest) tail round, all co-resident.
-__device__ __forceinline__ bool fri_tail_spin(volatile const unsigned long long *flag, unsigned long long want,
-                                              long long limit, volatile const uint64_t *abort_flag) {
-    const long long t0 = clock64();
-    while (*flag < want) {
-        if (abort_flag && *abort_flag != 0) return false;
-        if (clock64() - t0 > limit) return false;
-    }
-    return true;
-}
-__global__ void __launch_bounds__(MK_THREADS, 2) k_fri_tail(const __grid_constant__ FriTailArgs t) {
-    __shared__ uint64_t sm[MK_THREADS * 8];
-    __shared__ uint32_t s_sm[4];
-    __shared__ int s_ok;
-    const int tid = threadIdx.x;
-    const long long blk = blockIdx.x;
-    fe s_m = t.s_m0;
-    for (int i = 0; i < t.nrounds; i++) {
-        MerkleArgs a;
-        a.width = t.width0 >> i;
-        a.mode = 2;
-        merkle_shape(a);
-        const unsigned nblocks = (unsigned)(a.width / a.chunk);
-        if (blk >= nblocks) return;  // the rounds only get narrower: nothing left for this CTA
-        if (i > 0) {
-            // the challenge of this round: CTA 0 takes it from the host page and forwards it, the others
-            // watch the device flag (L2) instead of all polling across PCIe
-            if (tid == 0) {
-                const unsigned long long want = t.seq0 + (unsigned long long)i - 1;
-                volatile unsigned long long *bc = (volatile unsigned long long *)t.bcast;
-                bool ok;
-                if (blk == 0) {
-                    ok = fri_tail_spin((volatile const unsigned long long *)(t.host + 18), want, t.spin_limit, t.host + 19);
-                    if (ok) {
-                        __threadfence_system();
-                        const uint64_t lo = t.host[16], hi = t.host[17];
-                        bc[2] = lo;
-                        bc[3] = hi;
-                        __threadfence();
-                        bc[0] = want;
-                    } else {
-                        bc[1] = 1;                             // tell the others to give up as well
-                        __threadfence();
-                        if (t.host[19] == 0) t.host[20] = 1;  // (a timeout, not a host abort)
-                    }
-                } else {
-                    ok = fri_tail_spin(bc, want, t.spin_limit, (volatile const uint64_t *)(bc + 1));
-                }
-                if (ok) {
-                    __threadfence();
-                    const uint64_t lo = bc[2], hi = bc[3];
-                    s_sm[0] = (uint32_t)lo;
-                    s_sm[1] = (uint32_t)(lo >> 32);
-                    s_sm[2] = (uint32_t)hi;
-                    s_sm[3] = (uint32_t)(hi >> 32);
-                }
-                s_ok = ok ? 1 : 0;
-            }
-            __syncthreads();
-            if (!s_ok) return;
-            s_m = fe_make(s_sm[0], s_sm[1], s_sm[2], s_sm[3]);
-        }
-        a.tree = t.tree[i];
-        a.values = nullptr;
-        a.prev = i == 0 ? t.prev0 : t.layer[i - 1];
-        a.next = t.layer[i];
-        a.xinv = t.xinv[i];
-        a.s_m = s_m;
-        a.inv2_m = t.inv2_m;
-        a.ticket = nblocks > 1 ? t.ticket : nullptr;
-        a.root_out = const_cast<uint64_t *>(t.host);
-        a.root_seq = t.seq0 + (unsigned long long)i;
-        merkle_chunk_body(a, blk, nblocks, sm);
-        __syncthreads();  // sm and s_sm are reused by the next round
-    }
+    __shared__ int s_last;  // after sm: ptxas then places sm at offset 0, which its 128-bit accesses need
+    merkle_chunk_body(a, blockIdx.x, gridDim.x, sm, s_last);
 }
 
 __global__ void k_merkle_paths(uint64_t *out, const uint64_t *tree, long long n, int depth,
@@ -1071,25 +917,19 @@ static int launch_tile_variant(const TileArgs &a, cudaStream_t st) {
         const int rc = optin_smem(ntt_tile_kernel<LOGL, ELOG, C, FLAGS>, attr_done, smem);
         if (rc != SA_OK) return rc;
     }
-    static const bool pdl = !(getenv("SA_NTT_PDL") && atoi(getenv("SA_NTT_PDL")) == 0);
-    if (pdl) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)grid);
-        cfg.blockDim = dim3(P::THREADS);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        const int tpb = tiles_per_batch;
-        SA_CUDA(cudaLaunchKernelEx(&cfg, ntt_tile_kernel<LOGL, ELOG, C, FLAGS>, a, total, tpb));
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        return SA_OK;
-    }
-    ntt_tile_kernel<LOGL, ELOG, C, FLAGS><<<(unsigned)grid, P::THREADS, smem, st>>>(a, total, tiles_per_batch);
-    SA_LAUNCH_CHECK();
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid);
+    cfg.blockDim = dim3(P::THREADS);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    const int tpb = tiles_per_batch;
+    SA_CUDA(cudaLaunchKernelEx(&cfg, ntt_tile_kernel<LOGL, ELOG, C, FLAGS>, a, total, tpb));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
     return SA_OK;
 }
 template <int LOGL, int ELOG, int C>
@@ -1108,6 +948,7 @@ static int launch_tile(const TileArgs &a, cudaStream_t st) {
 
 // tile shape: register block (log2 elements per thread) and columns per tile; with -DSA_TUNE
 // the environment variables SA_NTT_ELOG / SA_NTT_C select a shape for tuning runs.
+#ifdef SA_TUNE
 static int g_tile_elog = -1, g_tile_c = -1;
 static void tile_config() {
     if (g_tile_elog >= 0) return;
@@ -1115,10 +956,11 @@ static void tile_config() {
     g_tile_elog = e ? atoi(e) : 0;
     g_tile_c = c ? atoi(c) : 0;
 }
+#endif
 template <int LOGL>
 static int launch_tile_shape(const TileArgs &a, cudaStream_t st) {
-    tile_config();
 #ifdef SA_TUNE
+    tile_config();
     if (LOGL >= 9 && g_tile_elog > 0) {
         if (g_tile_elog == 3 && g_tile_c == 8) return launch_tile<LOGL, 3, 8>(a, st);
         if (g_tile_elog == 3 && g_tile_c == 4) return launch_tile<LOGL, 3, 4>(a, st);
@@ -1134,12 +976,8 @@ static int launch_tile_shape(const TileArgs &a, cudaStream_t st) {
     if constexpr (LOGL >= 9) {
         // multi-GPU assembly (sa_ntt_multi): 8-column tiles store 128-byte instead of 64-byte segments to the
         // peers - the pass is bound by NVLink, not by the butterflies (8 GPUs, 16 x 2^20 incl. assembly: 0.468 ms
-        // against 0.665 ms with 4-column tiles, profiles/r02_notes.md); SA_NTT_PEER_C=4 for the comparison
-        static const int peer_c = [] {
-            const char *e = getenv("SA_NTT_PEER_C");
-            return e ? atoi(e) : 8;
-        }();
-        if ((a.npeer > 0 || a.mc_out != nullptr) && peer_c == 8) return launch_tile<LOGL, 4, 8>(a, st);
+        // against 0.665 ms with 4-column tiles, profiles/r02_notes.md)
+        if (a.npeer > 0 || a.mc_out != nullptr) return launch_tile<LOGL, 4, 8>(a, st);
         // (a LONE 2^20 transform is one partial wave per pass: 256 tiles on 2 x 148 slots, 108 SMs carry 8 columns
         // and 40 carry 4.  Seven-column tiles - 147 CTAs of 448 threads, one per SM, every SM the same 7 columns -
         // were built, emulated bit-exact and measured: 70 us against 60 us.  One 14-warp CTA per SM whose warps
@@ -1305,24 +1143,6 @@ int sa_push(void *const *dsts, int ndst, const void *src, size_t bytes, void *st
     const size_t n16 = bytes / 16;
     size_t grid = (n16 + 255) / 256;
     if (grid > (size_t)ctas) grid = (size_t)ctas;
-    static const int mode = [] {
-        const char *e = getenv("SA_PUSH_MODE");
-        return e ? atoi(e) : 0;
-    }();
-    if (mode == 2) {
-        size_t g = (bytes + PUSH_TMA_CHUNK - 1) / PUSH_TMA_CHUNK;
-        const size_t cap = (size_t)ctas * 4;  // one-warp CTAs with 32 KB of shared memory: several per SM
-        if (g > cap) g = cap;
-        k_push_tma<<<(unsigned)g, 32, 0, (cudaStream_t)stream>>>(a, (const char *)src, bytes);
-        SA_LAUNCH_CHECK();
-        return SA_OK;
-    }
-    if (mode == 1 && grid >= (size_t)ndst) {
-        grid -= grid % (size_t)ndst;
-        k_push_per_peer<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(a, (const uint4 *)src, n16);
-        SA_LAUNCH_CHECK();
-        return SA_OK;
-    }
     k_push<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(a, (const uint4 *)src, n16);
     SA_LAUNCH_CHECK();
     return SA_OK;
@@ -1948,8 +1768,7 @@ static unsigned int *get_ticket(cudaStream_t st) {
     return slot;  // nullptr: fall back to one more launch
 }
 static int merkle_reduce(MerkleArgs a, cudaStream_t st, uint64_t *root_host = nullptr, unsigned long long seq = 0) {
-    static const bool no_fuse = getenv("SA_MK_NO_FUSED_TOP") != nullptr;  // A/B switch for measurements
-    unsigned int *ticket = no_fuse ? nullptr : get_ticket(st);
+    unsigned int *ticket = get_ticket(st);
     // first launch handles the bottom level in a.mode, later launches continue from digests
     while (true) {
         merkle_shape(a);
@@ -2106,71 +1925,12 @@ static int wait_for_root(uint64_t *root_host, unsigned long long seq, cudaStream
     return SA_OK;
 }
 
-}  // extern "C"
-
-// ---- can the host talk to a RUNNING kernel?  (the persistent FRI tail depends on it) ----
-// Under tools that serialise launches (ncu / compute-sanitizer make a launch return only when the kernel has
-// finished; CUDA_LAUNCH_BLOCKING=1 does the same) a kernel that waits for the host would wait for ever, so the
-// tail is only used after this probe has passed once in the process: a one-thread kernel waits (at most
-// ~50 ms) for a flag the host sets right AFTER the launch call has returned.
-__global__ void k_host_probe(volatile uint64_t *page, long long limit) {
-    const long long t0 = clock64();
-    while (page[0] == 0 && clock64() - t0 < limit) {
-    }
-    page[1] = page[0] != 0 ? 1 : 2;
-    __threadfence_system();
-}
-static int g_tail_mode = -1;  // -1 not probed yet, 0 per-round launches, 1 persistent tail
-static std::mutex g_tail_mu;
-static bool fri_tail_allowed(cudaStream_t st) {
-    std::lock_guard<std::mutex> lock(g_tail_mu);
-    if (g_tail_mode >= 0) return g_tail_mode == 1;
-    g_tail_mode = 0;
-    // opt-in: measured on B200 (profiles/r02_notes.md, r02d) the persistent tail is no faster than one launch
-    // per round - the narrow rounds are blake2b dependency chains, not launch overhead
-    const char *e = getenv("SA_FRI_PERSISTENT");
-    if (!e || atoi(e) == 0) return false;
-    uint64_t *page = nullptr, *page_dev = nullptr;
-    if (cudaHostAlloc((void **)&page, 64, cudaHostAllocMapped) != cudaSuccess) {
-        cudaGetLastError();
-        return false;
-    }
-    page[0] = page[1] = 0;
-    bool ok = cudaHostGetDevicePointer((void **)&page_dev, page, 0) == cudaSuccess;
-    if (ok) {
-        k_host_probe<<<1, 1, 0, st>>>(page_dev, 100000000ll);
-        __atomic_store_n(&page[0], 1ull, __ATOMIC_RELEASE);  // only reaches a kernel that is running NOW
-        ok = cudaStreamSynchronize(st) == cudaSuccess && page[1] == 1;
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-    }
-    cudaFreeHost(page);
-    cudaGetLastError();
-    g_tail_mode = ok ? 1 : 0;
-    return ok;
-}
-// per (device, stream): ticket-like broadcast words of the tail kernel
-static std::map<std::pair<int, cudaStream_t>, unsigned long long *> g_bcast;
-static unsigned long long *get_bcast(cudaStream_t st) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
-    std::lock_guard<std::mutex> lock(g_ws_mu);
-    auto &slot = g_bcast[std::make_pair(dev, st)];
-    if (!slot && cudaMalloc((void **)&slot, 256) != cudaSuccess) {
-        slot = nullptr;
-        cudaGetLastError();
-    }
-    return slot;
-}
-
-extern "C" {
-
 int sa_fri_commit(void *layers, void *trees, const void *codeword, size_t n, int rounds,
                   const uint64_t offset[2], const uint64_t omega[2], sa_fri_challenge_fn challenge, void *user,
                   void *stream) {
     if (!host_is_pow2(n) || rounds < 1 || (n >> (rounds - 1)) < 1) return SA_ESIZE;
     cudaStream_t st = (cudaStream_t)stream;
-    // landing pad of the per-round root (8 words) + sequence number, written by the kernel itself; words
-    // 16.. carry the challenge the other way for the persistent tail (FriTailArgs::host)
+    // landing pad of the per-round root (8 words) + sequence number, written by the kernel itself
     static thread_local uint64_t *root_pinned = nullptr;
     static thread_local uint64_t *root_dev = nullptr;  // the same memory as the device addresses it
     static thread_local unsigned long long root_seq = 0;
@@ -2192,41 +1952,6 @@ int sa_fri_commit(void *layers, void *trees, const void *codeword, size_t n, int
     static const bool trace = getenv("SA_FRI_TRACE") != nullptr;  // per-round host timeline on stderr
     auto now = [] { return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     double t_mark = now();
-    // The narrow rounds (<= 2^FRI_TAIL_MAX_LOG leaves) run in ONE persistent launch when the host can talk to
-    // a running kernel; their x^-1 tables are fetched up front (building one synchronises the stream).
-    int tail_from = rounds;  // first round r (>= 1) whose tree has n >> r <= 2^FRI_TAIL_MAX_LOG leaves
-    for (int r = 1; r < rounds; r++)
-        if ((n >> r) <= ((size_t)1 << FRI_TAIL_MAX_LOG)) {
-            tail_from = r;
-            break;
-        }
-    std::vector<XinvPtr> tail_xinv;
-    unsigned int *tail_ticket = nullptr;
-    unsigned long long *tail_bcast = nullptr;
-    if (tail_from < rounds && rounds - tail_from <= FRI_TAIL_MAX_ROUNDS && fri_tail_allowed(st)) {
-        fe om_r = om;
-        for (int r = 1; r < rounds; r++) {  // round r folds with omega^(2^(r-1)) over n >> (r-1) points
-            if (r >= tail_from) {
-                XinvPtr x;
-                if ((rc = get_xinv(&x, om_r, n >> (r - 1), st)) != SA_OK) return rc;
-                tail_xinv.push_back(x);
-            }
-            om_r = fe_montmul(fe_to_mont(om_r), om_r);
-        }
-        tail_ticket = get_ticket(st);
-        tail_bcast = get_bcast(st);
-        if (!tail_ticket || !tail_bcast) tail_xinv.clear();
-    }
-    const bool use_tail = !tail_xinv.empty();
-    bool tail_running = false;
-    unsigned long long tail_seq0 = 0;
-    auto abort_tail = [&]() {
-        if (tail_running) {
-            __atomic_store_n(&root_pinned[19], 1ull, __ATOMIC_RELEASE);
-            cudaStreamSynchronize(st);
-            root_pinned[19] = 0;
-        }
-    };
     for (int r = 0; r < rounds; r++) {
         if (r == 0) {
             MerkleArgs a;
@@ -2238,89 +1963,34 @@ int sa_fri_commit(void *layers, void *trees, const void *codeword, size_t n, int
             if ((rc = merkle_reduce(a, st, root_dev, ++root_seq)) != SA_OK) return rc;
         }
         const double t_launched = now();
-        if ((rc = wait_for_root(root_pinned, root_seq, st)) != SA_OK) {
-            if (tail_running && root_pinned[20] != 0) g_last_error = "sa_fri_commit: the tail kernel timed out waiting for a challenge";
-            return rc;
-        }
+        if ((rc = wait_for_root(root_pinned, root_seq, st)) != SA_OK) return rc;
         const double t_synced = now();
         uint64_t alpha[2] = {0, 0};
         const int want = r != rounds - 1;
-        if (challenge(user, r, (const uint8_t *)root_pinned, alpha, want) != 0) {
-            abort_tail();
-            return SA_ECALLBACK;
-        }
+        if (challenge(user, r, (const uint8_t *)root_pinned, alpha, want) != 0) return SA_ECALLBACK;
         if (trace) {
             const double t_cb = now();
-            fprintf(stderr, "sa_fri_commit round %2d len %8zu: launch %.1f us, wait %.1f us, callback %.1f us%s\n", r, len,
-                    t_launched - t_mark, t_synced - t_launched, t_cb - t_synced, tail_running ? " (tail kernel)" : "");
+            fprintf(stderr, "sa_fri_commit round %2d len %8zu: launch %.1f us, wait %.1f us, callback %.1f us\n", r, len,
+                    t_launched - t_mark, t_synced - t_launched, t_cb - t_synced);
             t_mark = t_cb;
         }
         if (!want) break;
         // fold layer r into layer r+1 and build its tree: alpha / (2 offset), Montgomery form
         const fe s_m = fe_montmul(fe_montmul(fe_to_mont(fe_from_limbs(alpha)), inv2_m), oinv_m);
         uint8_t *next_tree = tree + 128 * len;  // this tree has 2 * len nodes of 64 bytes
-        if (tail_running) {
-            // the kernel is waiting for exactly this: s_m, then its sequence number (release order)
-            root_pinned[16] = (uint64_t)s_m.v[0] | ((uint64_t)s_m.v[1] << 32);
-            root_pinned[17] = (uint64_t)s_m.v[2] | ((uint64_t)s_m.v[3] << 32);
-            __atomic_store_n(&root_pinned[18], tail_seq0 + (unsigned long long)(r + 1 - tail_from) - 1, __ATOMIC_RELEASE);
-            ++root_seq;
-        } else if (use_tail && r + 1 == tail_from) {
-            FriTailArgs t;
-            memset(&t, 0, sizeof(t));
-            t.nrounds = rounds - tail_from;
-            t.width0 = (long long)(len / 2);
-            t.prev0 = cur;
-            fe *lo = layer_out;
-            uint8_t *tr = next_tree;
-            for (int i = 0; i < t.nrounds; i++) {
-                const size_t w = (len / 2) >> i;
-                t.layer[i] = lo;
-                t.tree[i] = (uint64_t *)tr;
-                t.xinv[i] = tail_xinv[i]->tab;
-                lo += w;
-                tr += 128 * w;
-            }
-            t.inv2_m = inv2_m;
-            t.s_m0 = s_m;
-            t.ticket = tail_ticket;
-            t.bcast = tail_bcast;
-            t.host = root_dev;
-            tail_seq0 = root_seq + 1;
-            t.seq0 = tail_seq0;
-            static const long long limit_ticks = [] {
-                const char *e = getenv("SA_FRI_TAIL_TIMEOUT_S");
-                const double sec = e ? atof(e) : 20.0;
-                return (long long)(sec * 2.0e9);
-            }();
-            t.spin_limit = limit_ticks;
-            root_pinned[19] = root_pinned[20] = 0;
-            SA_CUDA(cudaMemsetAsync(tail_bcast, 0, 64, st));
-            MerkleArgs shape;
-            shape.width = t.width0;
-            shape.mode = 2;
-            merkle_shape(shape);
-            const unsigned grid = (unsigned)(t.width0 / shape.chunk);
-            if (grid > (unsigned)FRI_TAIL_MAX_CTAS) return SA_ESIZE;  // (cannot happen: widths <= 2^16)
-            k_fri_tail<<<grid, MK_THREADS, 0, st>>>(t);
-            SA_LAUNCH_CHECK();
-            tail_running = true;
-            ++root_seq;
-        } else {
-            XinvPtr xinv;
-            if ((rc = get_xinv(&xinv, om, len, st)) != SA_OK) return rc;
-            MerkleArgs a;
-            memset(&a, 0, sizeof(a));
-            a.tree = (uint64_t *)next_tree;
-            a.width = (long long)(len / 2);
-            a.mode = 2;
-            a.prev = cur;
-            a.next = layer_out;
-            a.xinv = xinv->tab;
-            a.inv2_m = inv2_m;
-            a.s_m = s_m;
-            if ((rc = merkle_reduce(a, st, root_dev, ++root_seq)) != SA_OK) return rc;
-        }
+        XinvPtr xinv;
+        if ((rc = get_xinv(&xinv, om, len, st)) != SA_OK) return rc;
+        MerkleArgs a;
+        memset(&a, 0, sizeof(a));
+        a.tree = (uint64_t *)next_tree;
+        a.width = (long long)(len / 2);
+        a.mode = 2;
+        a.prev = cur;
+        a.next = layer_out;
+        a.xinv = xinv->tab;
+        a.inv2_m = inv2_m;
+        a.s_m = s_m;
+        if ((rc = merkle_reduce(a, st, root_dev, ++root_seq)) != SA_OK) return rc;
         cur = layer_out;
         layer_out += len / 2;
         tree = next_tree;
@@ -2331,11 +2001,6 @@ int sa_fri_commit(void *layers, void *trees, const void *codeword, size_t n, int
         oinv_m = fe_montmul(oinv_m, oinv_m);  // (offset^2)^-1, stays in Montgomery form
     }
     return SA_OK;
-}
-
-int sa_fri_tail_mode(void) {
-    std::lock_guard<std::mutex> lock(g_tail_mu);
-    return g_tail_mode;
 }
 
 size_t sa_cache_limit(size_t bytes) {

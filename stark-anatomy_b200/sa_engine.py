@@ -62,7 +62,6 @@ SYMBOLS = [
     ("sa_fri_fold", _ci, [_vp, _vp, _sz, _u64p, _u64p, _u64p, _vp]),
     ("sa_fri_round", _ci, [_vp, _vp, _vp, _sz, _u64p, _u64p, _u64p, _vp]),
     ("sa_fri_commit", _ci, [_vp, _vp, _vp, _sz, _ci, _u64p, _u64p, _vp, _vp, _vp]),
-    ("sa_fri_tail_mode", _ci, []),
     ("sa_cache_limit", _sz, [_sz]),
     ("sa_cache_bytes", _sz, []),
     ("sa_release_workspaces", _ci, []),
